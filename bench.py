@@ -10,6 +10,7 @@ statistics -> Umeyama -> compose), rmcl_ros/src/nodes/micp_localization.cpp:899-
 N > 1 (torchrun): poses are sharded, one pose (one sensor) per GPU, map replicated, no data-path collective ("weak" scaling).
 
   python bench.py --gpus 1 --steps 200 --warmup 20
+  python bench.py --gpus 1 --steps 200 --warmup 20 --dump-outputs /tmp/out    # + the last timed step's result as .npy files
   python bench.py --impl reference ...      # the reference's CPU path (oracle port: Embree/rmagine are not buildable here) on the host cores
 """
 import argparse
@@ -40,7 +41,23 @@ def parse():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary workloads (C3 particle filter, v1 batched correct)")
     ap.add_argument("--faces", type=int, default=N_FACES)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned (the correctOnce result: "
+                    "new pose, pose delta, merged statistics) to DIR/<name>.npy; same arguments, same inputs, so two builds compare output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
+
+
+def dump_outputs(path, records):
+    """One DIR/<record>_<field>.npy per field of each returned record: float32 fields as they are, integer fields (n_meas, stamp) as float64."""
+    os.makedirs(path, exist_ok=True)
+    for name, rec in records.items():
+        for field in rec.dtype.names:
+            v = np.asarray(rec[field])
+            np.save(os.path.join(path, f"{name}_{field}.npy"), v if v.dtype == np.float32 else v.astype(np.float64))
 
 
 def rank_pose(synth, rank):
@@ -298,6 +315,8 @@ def main():
         inflight -= 1
     launches = rmcl_b200.kernel_launch_count() - launches0
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"Tom_new": Tn, "T_onew_oold": Td, "C_merged": Cm})
     step_ms = np.array([a.elapsed_time(b) for a, b in ev], np.float64)
     dev_ms = float(step_ms.sum())
 
